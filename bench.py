@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- events/s through divide_rounds + decide_fame (BASELINE.json's metric).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload c3]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload c3] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over the whole synthetic trace of the workload: for every
 chunk of the pinned call schedule, `divide_rounds(chunk)` then `decide_fame()` (swirld.py:325-327),
@@ -25,8 +25,12 @@ starting from an engine whose consensus state was cleared.  Workloads (BASELINE.
             duration (CUDA events on the engine's stream) against MEASURED_PEAKS.json hbm_gbs.
 `roofline_can_see`: the same for the can_see kernel family k_cs_* (B1(M) = 12M + 12 bytes per event).
 `cpu_baseline` / --impl reference: the literal C restatement oracle/ (kind "port"), single-threaded per node-view
-            like the reference (README.md:27-28), plus -- where baseline/_ref holds the staged reference files --
+            like the reference (README.md:27-28), plus -- where SWIRLD_REFERENCE names a checkout of the reference --
             the UNMODIFIED Python reference timed on a prefix of the same trace (`python_reference`).
+`--dump-outputs DIR`: what the last timed step computed (rank 0) as DIR/<name>.npy, float32 (float64 for event
+            indices past 2**24 and for the sample index), at most 64 MiB in all: round, witness, famous per event --
+            a fixed seeded sample of the events (sample_index.npy) when the whole columns would not fit -- and the
+            witness_table and consensus rounds.  The traces are seeded, so the same arguments give the same inputs.
 
 N > 1, one process per GPU (torchrun):
   c1-c3 (M <= 64): independent node-views ("replicas", DESIGN.md section 6: a round step costs less than any
@@ -44,6 +48,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -135,7 +140,7 @@ class ClockSampler:
 def make_trace(wl, seed):
     from swirld_b200 import traces
     gen = wl.get("gen", "gossip")
-    cache = "/tmp/swirld_trace_%s_M%d_N%d_s%d.npz" % (gen, wl["M"], wl["N"], seed)
+    cache = os.path.join(tempfile.gettempdir(), "swirld_trace_%s_M%d_N%d_s%d.npz" % (gen, wl["M"], wl["N"], seed))
     if os.path.exists(cache):
         try:
             z = np.load(cache)
@@ -187,22 +192,20 @@ def reference_sample_events(wl, steps):
 
 
 def python_reference_sample(tr, wl):
-    """The UNMODIFIED Python reference (staged under baseline/_ref by __graft_entry__.build()) on a prefix of the
-    trace: events/s through its own divide_rounds + decide_fame.  None when the files did not travel."""
-    ref = os.path.join(ROOT, "baseline", "_ref")
-    if not os.path.isfile(os.path.join(ref, "swirld.py")):
-        return None
-    os.environ["SWIRLD_REFERENCE"] = ref
+    """The UNMODIFIED Python reference (the checkout SWIRLD_REFERENCE names) on a prefix of the trace: events/s
+    through its own divide_rounds + decide_fame.  None without one."""
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
+    import ref_harness as rh
+    if not rh.reference_available():
+        return None
     try:
-        import ref_harness as rh
         M = wl["M"]
         n = min(tr.N, max(2000, 3 * M, int(12 * 5.6e3 * (64.0 / max(M, 8)) ** 2)))     # ~10-40 s of CPython; past the M root events
         K = min(wl["K"], 2000) if n > 2000 else wl["K"]
         r = rh.run_reference(tr.slice(0, n), K)
         s = r["t_divide_rounds"] + r["t_decide_fame"]
         return {"value": n / s, "unit": "events/s", "cores": 1, "kind": "reference-python",
-                "sample": "first %d events, K=%d, unmodified swirld.py (baseline/_ref) through oracle/ref_harness.py, "
+                "sample": "first %d events, K=%d, unmodified swirld.py through oracle/ref_harness.py, "
                           "divide_rounds %.2f s + decide_fame %.2f s (find_order %.2f s not counted)" % (
                               n, K, r["t_divide_rounds"], r["t_decide_fame"], r["t_find_order"])}
     except Exception as ex:      # the reference arm must not take the bench down
@@ -286,6 +289,7 @@ def stream_leg(local_rank, cases=((4, 2000, 1), (4, 2000, 50), (64, 20000, 3))):
     from swirld_b200.traces import chunks
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     import oracle as orc
+    import ref_harness as rh
     out = []
     for M, N, K in cases:
         tr = traces.gossip(M, N, 1)
@@ -311,11 +315,8 @@ def stream_leg(local_rank, cases=((4, 2000, 1), (4, 2000, 50), (64, 20000, 3))):
             e.close()
         same = all(np.array_equal(np.asarray(o[k]), np.asarray(res[k])) for k in ("round", "witness_table", "famous", "consensus", "transactions"))
         pyref = None
-        ref = os.path.join(ROOT, "baseline", "_ref")
-        if os.path.isfile(os.path.join(ref, "swirld.py")):
-            os.environ["SWIRLD_REFERENCE"] = ref
+        if rh.reference_available():
             try:
-                import ref_harness as rh
                 npre = min(N, 6000 if M >= 64 else 2000)
                 r = rh.run_reference(tr.slice(0, npre), K)
                 pyref = npre / (r["t_divide_rounds"] + r["t_decide_fame"] + r["t_find_order"])
@@ -357,6 +358,32 @@ def connect_peers(eng, dist, rank, world):
     parts = [None] * world
     dist.all_gather_object(parts, mine)
     eng.peer_connect(rank, world, b"".join(parts))
+
+
+# --------------------------------------------------------------------------- output dump
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, n_events, per_event, tables):
+    """per_event: name -> column of n_events values; tables: name -> array (event indices, round numbers).  Writes
+    each as out_dir/<name>.npy, float32 while event indices stay exact in it, else float64.  When the columns do not
+    fit in DUMP_BYTES beside the tables, the same seeded sample of events is taken from each, its indices in
+    sample_index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    fdt = np.dtype(np.float32 if n_events <= 1 << 24 else np.float64)
+    out = {k: np.asarray(v).astype(fdt) for k, v in tables.items()}
+    room = DUMP_BYTES - (64 << 10) - sum(v.nbytes for v in out.values())      # (64 KiB for the .npy headers)
+    row = len(per_event) * fdt.itemsize
+    if n_events * row > room:
+        keep = room // (row + 8)
+        if keep < 1:
+            raise SystemExit("bench.py: --dump-outputs: the tables alone exceed %d bytes" % DUMP_BYTES)
+        idx = np.sort(np.random.default_rng(20240917).choice(n_events, keep, replace=False))
+        out["sample_index"] = idx.astype(np.float64)
+        per_event = {k: np.asarray(v)[idx] for k, v in per_event.items()}
+    out.update({k: np.asarray(v).astype(fdt) for k, v in per_event.items()})
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 # --------------------------------------------------------------------------- GPU arm
@@ -465,6 +492,9 @@ def bench_ours(args, wl, rank, world, local_rank):
     st1 = eng.stats()
     got_round, got_wit, got_fam = eng.rounds(), eng.witness_flags(), eng.famous()
     check = (int(got_round.astype(np.int64).sum()), int(eng.max_round), int(len(eng.consensus())))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, N, {"round": got_round, "witness": got_wit, "famous": got_fam},
+                     {"witness_table": eng.witness_table(), "consensus": eng.consensus()})
 
     # ---- several node-views per launch (M <= 64: SURVEY.md section 8f-3): B independent views (own traces) advanced by
     #      sw_batch_divide_rounds, aggregate events/s over all views, device-timed on the first view's stream
@@ -672,7 +702,13 @@ def main():
     ap.add_argument("--views", default="", help="comma list of view counts B for the multi-view leg (M <= 64), e.g. 1,8,32")
     ap.add_argument("--views-events", type=int, default=0, help="events per view in the multi-view leg (default: the workload's)")
     ap.add_argument("--no-python-reference", action="store_true")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (at most 64 MiB)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU arm computed; --impl reference has no such step")
     wl = dict(WORKLOADS[args.workload])
     if args.events:
         wl["N"] = args.events

@@ -44,13 +44,36 @@ SPECS = {
     "g4_m9_n6000_join3000_s77_k2500": ("late_joiner", dict(M=9, N=6000, join_at=3000, seed=77), 2500, None),
 }
 
+
+# small spot checks of the oracle against the reference (tests/test_oracle_golden.py): for each (M, N, K, seed)
+# one gossip trace and one adversarial trace with at least four members
+SPOT_CASES = [(4, 600, 1, 11), (5, 900, 13, 12), (16, 3000, 250, 13)]
+
+
+def spot_names(M, N, K, seed):
+    return ["spot_g1_m%d_n%d_s%d_k%d" % (M, N, seed, K), "spot_g2_m%d_n%d_s%d_k%d" % (max(M, 4), N, seed, K)]
+
+
+SPOTS = {}
+for _M, _N, _K, _seed in SPOT_CASES:
+    _g1, _g2 = spot_names(_M, _N, _K, _seed)
+    SPOTS[_g1] = ("gossip", dict(M=_M, N=_N, seed=_seed), _K, None)
+    SPOTS[_g2] = ("adversarial", dict(M=max(_M, 4), N=_N, seed=_seed, p_cross=0.05, p_stale=0.3), _K, None)
+
+# node traces recorded from one gossip simulation of tests/node_sim.py (4 nodes, 400 turns, seed 5: real keys and
+# clock timestamps, so the traces themselves are stored), replayed through the reference with each node's own
+# call schedule
+NODE_SIM = ["node_sim_n4_t400_node0", "node_sim_n4_t400_node1"]
+# the same for every node of one run of the reference's own driver, swirld.test(4, 300), over bind(swirld.Node)
+DROP_IN = ["drop_in_n4_t300_node%d" % i for i in range(4)]
+
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))),
                           "tests", "golden")
 
 
 def make_trace(name):
     from swirld_b200 import traces
-    gen, kw, K, stake = SPECS[name]
+    gen, kw, K, stake = SPECS[name] if name in SPECS else SPOTS[name]
     return getattr(traces, gen)(**kw), K, stake
 
 

@@ -1,12 +1,12 @@
-"""Tier-0 oracle: drive the UNMODIFIED reference (/root/reference/swirld.py)
+"""Tier-0 oracle: drive the UNMODIFIED reference (swirld.py of Lapin0t/py-swirld)
 through its own hot-path methods on an index-space trace.
 
-TEST INFRASTRUCTURE ONLY.  Works only where /root/reference is mounted (this
-container, not the GPU box); used by `oracle/make_golden.py` to produce the
-fixtures under `tests/golden/` and by the CPU tests that pin the C restatement
-(`oracle/swirld_oracle.c`) when the reference is present.  Nothing is copied
-from the reference: it is imported from where it lies, behind the `pysodium`
-shim in `oracle/pysodium_shim/`.
+TEST INFRASTRUCTURE ONLY.  Works only where the environment variable
+SWIRLD_REFERENCE names a checkout of the reference; used by
+`oracle/make_golden.py` to produce the fixtures under `tests/golden/` (which the
+tests compare against) and by bench.py's optional timing of the reference.
+Nothing is copied from the reference: it is imported from where it lies,
+behind the `pysodium` shim in `oracle/pysodium_shim/`.
 
 Recipe (SURVEY.md Appendix A.2): one `Node`, the state its constructor made for
 its own root event thrown away, events fed with integer ids through
@@ -25,14 +25,11 @@ from collections import defaultdict
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.environ.get("SWIRLD_REFERENCE", "/root/reference")
-if not os.path.isfile(os.path.join(REF, "swirld.py")):
-    # the files __graft_entry__.build() staged (git-ignored; they travel to the GPU box with gpurun)
-    REF = os.path.join(os.path.dirname(HERE), "baseline", "_ref")
+REF = os.environ.get("SWIRLD_REFERENCE", "")
 
 
 def reference_available() -> bool:
-    return os.path.isfile(os.path.join(REF, "swirld.py"))
+    return bool(REF) and os.path.isfile(os.path.join(REF, "swirld.py"))
 
 
 def load_reference():
@@ -42,7 +39,7 @@ def load_reference():
         sys.path.insert(0, shim)
     if REF not in sys.path:
         sys.path.insert(1, REF)
-    import swirld  # noqa: the reference, from /root/reference
+    import swirld  # noqa: the reference, from SWIRLD_REFERENCE
     return swirld
 
 

@@ -49,6 +49,31 @@ def replay_oracle(tr, sizes):
     return o.results()
 
 
-def replay_reference(tr, sizes):
-    import ref_harness as rh
-    return rh.run_reference(tr, sizes)
+def replay_node(g, engine_cls=None):
+    """A bound node fed a recorded node trace (fixture `g`: trace columns + call schedule) the way a host feeds it:
+    its own root from `new_event`, then per call the new events through `add_event` and one (divide_rounds,
+    decide_fame, find_order) triple.  Ids and member keys are synthetic; the engine reads parents, creator, time and
+    signature only."""
+    M, sizes = int(g["M"]), g["sizes"].tolist()
+    pks = [bytes([m]) * 32 for m in range(M)]
+    ids = [i.to_bytes(8, "little") for i in range(len(g["p0"]))]
+
+    def event(i):
+        p = () if g["p0"][i] < 0 else (ids[g["p0"][i]], ids[g["p1"][i]])
+        return host_sim.Event(None, p, float(g["t"][i]), pks[g["creator"][i]], bytes(g["sig"][i]))
+
+    class Replay:
+        def new_event(self, d, p):
+            return ids[0], event(0)
+
+    assert sizes[0] == 1
+    nd = bound_class(Replay, engine_cls)((pks[g["creator"][0]], b""), {}, M, {pk: 1 for pk in pks})
+    first = 1
+    for s in sizes[1:]:
+        for i in range(first, first + s):
+            nd.add_event(ids[i], event(i))
+        nd.divide_rounds(ids[first:first + s])
+        nd.find_order(nd.decide_fame())
+        first += s
+    return nd
+

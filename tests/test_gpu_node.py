@@ -43,22 +43,13 @@ def test_simulation_over_the_gpu_engine(n_nodes, turns, cap):
 
 
 def test_reference_node_bound_to_the_gpu_engine():
-    """Where the reference's files are available (baseline/_ref travels to the GPU box): `swirld.test` over
-    bind(swirld.Node) on the real engine, each node against the oracle's replay of its own trace and schedule."""
-    import contextlib
-    import io
-    import ref_harness as rh
-    if not rh.reference_available():
-        pytest.skip("reference files not staged")
-    from swirld_b200 import node as gnode
-    swirld = rh.load_reference()
-    saved = swirld.Node
-    try:
-        swirld.Node = gnode.bind(saved)
-        with contextlib.redirect_stdout(io.StringIO()):
-            nodes = swirld.test(4, 250)
-    finally:
-        swirld.Node = saved
-    for nd in nodes:
-        tr, sizes = node_sim.node_trace(nd)
-        assert_same(node_sim.replay_oracle(tr, sizes), node_sim.node_results(nd), KEYS, "bind(swirld.Node) vs oracle replay")
+    """What the reference's own driver fed every node of `swirld.test(4, 300)` over bind(swirld.Node) (gs.DROP_IN,
+    recorded by oracle/make_golden.py), fed again to a node bound to the real engine: each node against the reference's
+    replay of its own trace and schedule."""
+    import golden_specs as gs
+    from util import load_golden
+    for name in gs.DROP_IN:
+        g = load_golden(name)
+        nd = node_sim.replay_node(g)
+        assert node_sim.node_trace(nd)[1] == g["sizes"].tolist()
+        assert_same(g, node_sim.node_results(nd), KEYS, name + ": bind(swirld.Node) on the GPU vs reference")

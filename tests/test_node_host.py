@@ -1,14 +1,16 @@
 """The bound node's host logic on CPU: a gossip simulation (real Ed25519 signatures, BLAKE2b ids, random peers)
-runs over `bind(host)` with the oracle standing in for the device -- over the tests' own host everywhere, and over
-the reference's `swirld.Node` itself (its `sync` / `ask_sync` / `new_event` / `main` inherited unchanged) where the
-reference is available; every node's state must equal a replay of its own arrival trace and call schedule through
-the oracle and through the unmodified reference."""
+runs over `bind(host)` with the oracle standing in for the device, over the tests' own host; every node's state must
+equal a replay of its own arrival trace and call schedule through the oracle.  Node traces recorded from this
+simulation and from the reference's own driver over `bind(swirld.Node)` are replayed against the unmodified
+reference's results on them (tests/golden)."""
+import numpy as np
 import pytest
 
+import golden_specs as gs
 import node_sim
-import ref_harness as rh
 from oracle_engine import OracleEngine
-from util import assert_same
+from swirld_b200.traces import Trace
+from util import assert_same, load_golden
 
 KEYS = ["round", "famous", "consensus", "transactions"]
 
@@ -51,32 +53,28 @@ def test_each_node_matches_oracle_replay(sim):
         assert_same(node_sim.replay_oracle(tr, sizes), node_sim.node_results(nd), KEYS, "node vs oracle replay")
 
 
-@pytest.mark.skipif(not rh.reference_available(), reason="reference not mounted (GPU box)")
-def test_each_node_matches_reference_replay(sim):
-    for nd in sim[:2]:
-        tr, sizes = node_sim.node_trace(nd)
-        assert_same(node_sim.replay_reference(tr, sizes), node_sim.node_results(nd), KEYS, "node vs reference replay")
+def test_each_node_matches_reference_replay():
+    """Node traces and call schedules recorded from one run of this simulation, with the reference's replay of each
+    (gs.NODE_SIM, recorded by oracle/make_golden.py): the oracle's replay must reproduce it.  Every live node is tied
+    to the oracle's replay by test_each_node_matches_oracle_replay."""
+    for name in gs.NODE_SIM:
+        g = load_golden(name)
+        tr = Trace(int(g["M"]), g["p0"], g["p1"], g["creator"], g["t"], g["sig"], name)
+        assert_same(g, node_sim.replay_oracle(tr, g["sizes"].tolist()), KEYS, name + ": oracle replay vs reference replay")
 
 
-@pytest.mark.skipif(not rh.reference_available(), reason="reference not available")
 def test_drop_in_for_the_reference_drivers():
-    """`swirld.Node = bind(swirld.Node)` before `swirld.test(...)`: the reference's own driver, main loop, sync and
-    event code run unchanged (inherited) over the GPU-backed consensus state (SURVEY.md section 8b)."""
-    import contextlib
-    import io
-    swirld = rh.load_reference()
-    saved = swirld.Node
-    try:
-        swirld.Node = node_sim.bound_class(saved, OracleEngine)
-        assert swirld.Node.sync is saved.sync and swirld.Node.main is saved.main and swirld.Node.new_event is saved.new_event
-        with contextlib.redirect_stdout(io.StringIO()):
-            nodes = swirld.test(4, 300)
-    finally:
-        swirld.Node = saved
-    assert min(len(n.transactions) for n in nodes) > 5
-    for nd in nodes:       # each node equals the reference's replay of its own trace + schedule
+    """`swirld.Node = bind(swirld.Node)` before `swirld.test(4, 300)`: what the reference's own driver, main loop and
+    sync fed every node (its arrival trace and call schedule, gs.DROP_IN, recorded by oracle/make_golden.py) is fed
+    again to a bound node; its state must equal the reference's replay of the same trace and schedule."""
+    for name in gs.DROP_IN:
+        g = load_golden(name)
+        nd = node_sim.replay_node(g, OracleEngine)
         tr, sizes = node_sim.node_trace(nd)
-        assert_same(node_sim.replay_reference(tr, sizes), node_sim.node_results(nd), KEYS, "drop-in node vs reference")
+        assert sizes == g["sizes"].tolist()
+        assert all(np.array_equal(getattr(tr, k), g[k]) for k in ("p0", "p1", "creator", "t", "sig"))
+        assert len(nd.transactions) > 5
+        assert_same(g, node_sim.node_results(nd), KEYS, name + ": drop-in node vs reference")
 
 
 def test_forked_events_are_dropped_not_fatal():
