@@ -138,10 +138,36 @@ int sw_debug_counters(sw_engine *e, int64_t *out16, int clear);
  * batch; a cycle returns SW_E_ARG like toposort's ValueError), validated like sw_append validates (unknown parent,
  * parent shape, fork -- such an event, and whatever depends on it, is skipped: index -1), appended by ONE sw_append in
  * that order and entered in the engine's id -> index map.  index_out[i] = arrival index of input event i.  Returns
- * the number of events appended.  Signature checks (Ed25519) stay with the caller (libsodium, out of scope). */
+ * the number of events appended.  Signature and id checks are left to the caller: sw_ingest_verified makes them. */
 int sw_ingest(sw_engine *e, int n, const uint8_t *ids, const uint8_t *p0_ids, const uint8_t *p1_ids,
               const int32_t *creator, const double *t, const uint8_t *sig, int32_t *index_out);
 int sw_lookup(sw_engine *e, int n, const uint8_t *ids, int32_t *index_out);   /* id -> arrival index, -1 unknown */
+
+/* ---- is_valid_event's crypto checks (swirld.py:97-103) on the GPU.
+ * Public keys of the M members, 32 bytes each, in member order (Event.c; the stake dict's keys).  Decoded and checked
+ * once; tables for verification (48 KB per member) built on the device.  Returns the number of members whose key
+ * libsodium would reject (small order, non-canonical, not on the curve): no signature by such a member ever verifies.
+ * Keys survive sw_reset / sw_rewind; they are not part of the sw_save file (call again after sw_load). */
+int sw_set_member_keys(sw_engine *e, const uint8_t *pk);
+
+/* The two checks for n events:
+ *  msg  = concatenated dumps(ev[:-1]) (the signed bytes), msg_off[n+1] int64 offsets (event i: [msg_off[i], msg_off[i+1]));
+ *  wire = concatenated dumps(ev)      (the hashed bytes), wire_off[n+1];
+ *  sig  = n x 64 (Event.s), ids = n x 32, creator = member index.
+ * status_out[i]: bit 0 = crypto_sign_verify_detached(sig, msg, pk[creator]) succeeds (libsodium's verdict exactly);
+ * bit 1 = BLAKE2b-256(wire) == ids[i].  A creator outside [0, M) gives bit 0 = 0.  The engine checks the 64 bytes of
+ * `sig` -- the column sw_append stores, which the coin and the whitening read; the caller is responsible for msg and
+ * wire being the serialisation of that same event.  Changes no engine state.  SW_E_ARG before sw_set_member_keys.
+ * Returns the number of events with status 3. */
+int sw_verify(sw_engine *e, int n, const int32_t *creator, const uint8_t *sig, const uint8_t *msg, const int64_t *msg_off,
+              const uint8_t *ids, const uint8_t *wire, const int64_t *wire_off, uint8_t *status_out);
+
+/* sw_ingest with the crypto checks of is_valid_event: the new events of the batch (ids the engine does not know) are
+ * verified first; one whose status is not 3 is rejected like a shape- or fork-invalid one -- index -1, and everything
+ * that hangs below it is rejected too (swirld.py:133-136).  Columns as in sw_ingest and sw_verify. */
+int sw_ingest_verified(sw_engine *e, int n, const uint8_t *ids, const uint8_t *p0_ids, const uint8_t *p1_ids,
+                       const int32_t *creator, const double *t, const uint8_t *sig, const uint8_t *msg,
+                       const int64_t *msg_off, const uint8_t *wire, const int64_t *wire_off, int32_t *index_out);
 
 /* ---- checkpoint / resume (the reference keeps its state in memory only and uses pickle on the wire, swirld.py:129,160):
  * the engine's whole state -- event columns, can_see table, rounds, witness / fame tables, order -- as one binary file

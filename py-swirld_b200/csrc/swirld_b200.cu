@@ -9,6 +9,7 @@
 #include "swirld_rcluster.cuh"
 #include "swirld_wide.cuh"
 #include "swirld_stream.cuh"
+#include "swirld_verify.cuh"
 
 #include <cstdlib>
 #include "../../include/swirld_b200.h"
@@ -126,6 +127,14 @@ struct sw_engine {
     std::vector<TimedSpan> spans;
     std::vector<cudaEvent_t> pool;
     std::unordered_map<Id32, int32_t, Id32Hash> ids;     // sw_ingest: event id -> arrival index
+    // signature / id checks (swirld_verify.cuh): member keys, their comb tables (+ B's), the inputs of the last check
+    bool keys_set = false;
+    uint8_t *d_vpk = nullptr, *d_vkeyok = nullptr;
+    swv::Point *d_vbase = nullptr;
+    swv::Precomp *d_vtab = nullptr;
+    struct VBuf { void *p = nullptr; size_t cap = 0; };
+    VBuf vbuf[9];
+    int v_grid = 0;               // CTAs of k_verify that fit the device at once
     sw_stats_t stats{};
     std::string err;
 };
@@ -699,6 +708,9 @@ void sw_destroy(sw_engine *e) {
                     e->d_batch_ev, e->d_batch_seg, e->d_perm, e->d_ts, e->d_key, e->d_seg_start, e->d_seg_fw,
                     e->d_seg_nf, e->d_seg_white, e->d_rounds_in, e->d_plan, e->d_flush, e->d_rsg, e->d_rccont};
     for (void *p : ptrs) if (p) cudaFree(p);
+    void *vptrs[] = {e->d_vpk, e->d_vkeyok, e->d_vbase, e->d_vtab};
+    for (void *p : vptrs) if (p) cudaFree(p);
+    for (auto &b : e->vbuf) if (b.p) cudaFree(b.p);
     if (e->h_scal) cudaFreeHost(e->h_scal);
     if (e->h_newc) cudaFreeHost(e->h_newc);
     if (e->h_height) cudaFreeHost(e->h_height);
@@ -1178,10 +1190,12 @@ int sw_flush_l2(sw_engine *e, int64_t bytes) {
     return SW_OK;
 }
 
-// ---- ingest: what Node.sync does between the wire and divide_rounds (swirld.py:129-136, utils.py:8-21), natively
-int sw_ingest(sw_engine *e, int n, const uint8_t *ids, const uint8_t *p0_ids, const uint8_t *p1_ids,
-              const int32_t *creator, const double *t, const uint8_t *sig, int32_t *index_out) {
-    if (!e || n < 0 || (n > 0 && (!ids || !p0_ids || !p1_ids || !creator || !t || !sig || !index_out))) return fail(e, SW_E_ARG, "bad argument");
+// ---- ingest: what Node.sync does between the wire and divide_rounds (swirld.py:129-136, utils.py:8-21), natively.
+// rejected (optional): input events that failed a check made before (the crypto checks of sw_ingest_verified); they
+// are skipped like a shape- or fork-invalid event, and so is whatever hangs below them.
+namespace {
+int ingest_impl(sw_engine *e, int n, const uint8_t *ids, const uint8_t *p0_ids, const uint8_t *p1_ids,
+                const int32_t *creator, const double *t, const uint8_t *sig, const uint8_t *rejected, int32_t *index_out) {
     auto key = [](const uint8_t *p) { Id32 k; memcpy(k.data(), p, 32); return k; };
     const Id32 zero{};
     // 1. which events are new, and where each new id sits in the batch
@@ -1236,7 +1250,7 @@ int sw_ingest(sw_engine *e, int n, const uint8_t *ids, const uint8_t *p0_ids, co
     for (int i : order) {
         const int c = creator[i];
         int a, b;
-        if (c < 0 || c >= e->M || !resolve(i, 0, a) || !resolve(i, 1, b)) continue;
+        if ((rejected && rejected[i]) || c < 0 || c >= e->M || !resolve(i, 0, a) || !resolve(i, 1, b)) continue;
         if (a < 0 && b < 0) { if (head[c] >= 0) continue; }                         // a second root: fork
         else if (a < 0 || b < 0 || creator_of(a) != c || creator_of(b) == c || head[c] != a) continue;   // swirld.py:104-108 + fork-free
         if (next_index >= e->cap) return fail(e, SW_E_CAPACITY, "capacity_events=%d exceeded", e->cap);
@@ -1259,6 +1273,147 @@ int sw_ingest(sw_engine *e, int n, const uint8_t *ids, const uint8_t *p0_ids, co
     for (int i = 0; i < n; i++)
         if (index_out[i] < 0) { auto it = e->ids.find(key(ids + (size_t)32 * i)); index_out[i] = it == e->ids.end() ? -1 : it->second; }
     return m;
+}
+}  // namespace
+
+int sw_ingest(sw_engine *e, int n, const uint8_t *ids, const uint8_t *p0_ids, const uint8_t *p1_ids,
+              const int32_t *creator, const double *t, const uint8_t *sig, int32_t *index_out) {
+    if (!e || n < 0 || (n > 0 && (!ids || !p0_ids || !p1_ids || !creator || !t || !sig || !index_out))) return fail(e, SW_E_ARG, "bad argument");
+    return ingest_impl(e, n, ids, p0_ids, p1_ids, creator, t, sig, nullptr, index_out);
+}
+
+// ---- is_valid_event's crypto checks (swirld.py:97-103) on the device: swirld_verify.cuh
+int sw_set_member_keys(sw_engine *e, const uint8_t *pk) {
+    if (!e || !pk) return fail(e, SW_E_ARG, "bad argument");
+    CK(cudaSetDevice(e->device));
+    const int M = e->M;
+    if (!e->d_vtab) {
+        CK(dalloc(&e->d_vpk, (size_t)32 * M));
+        CK(dalloc(&e->d_vkeyok, (size_t)M + 1));
+        CK(dalloc(&e->d_vbase, (size_t)M + 1));
+        CK(dalloc(&e->d_vtab, (size_t)(M + 1) * swv::COMB_ENTRIES));
+    }
+    e->keys_set = false;
+    CK(cudaMemcpyAsync(e->d_vpk, pk, (size_t)32 * M, cudaMemcpyHostToDevice, e->stream));
+    k_verify_keys<<<(M + 1 + 127) / 128, 128, 0, e->stream>>>(e->d_vpk, M, e->d_vbase, e->d_vkeyok);
+    k_verify_table<<<((M + 1) * 64 + 127) / 128, 128, 0, e->stream>>>(e->d_vbase, e->d_vkeyok, M, e->d_vtab);
+    CK(cudaGetLastError());
+    std::vector<uint8_t> ok((size_t)M + 1);
+    CK(cudaMemcpyAsync(ok.data(), e->d_vkeyok, (size_t)M + 1, cudaMemcpyDeviceToHost, e->stream));
+    CK(cudaStreamSynchronize(e->stream));
+    e->stats.kernel_launches += 2;
+    e->stats.h2d_bytes += (int64_t)32 * M;
+    e->stats.d2h_bytes += M + 1;
+    if (!ok[M]) return fail(e, SW_E_CUDA, "sw_set_member_keys: the base point did not decode");
+    e->keys_set = true;
+    int bad = 0;
+    for (int m = 0; m < M; m++) bad += ok[m] == 0;
+    return bad;
+}
+
+namespace {
+// the engine's grow-only scratch slot `slot`, at least `bytes` long
+void *scratch(sw_engine *e, int slot, size_t bytes) {
+    auto &b = e->vbuf[slot];
+    bytes = std::max<size_t>(bytes, 16);
+    if (bytes > b.cap) {
+        if (b.p) cudaFree(b.p);
+        b.p = nullptr; b.cap = 0;
+        if (cudaMalloc(&b.p, bytes + bytes / 4) != cudaSuccess) { b.p = nullptr; return nullptr; }
+        b.cap = bytes + bytes / 4;
+    }
+    return b.p;
+}
+
+// device copy of a host buffer, in scratch slot `slot`
+extern "C++" template <typename T>
+int upload(sw_engine *e, int slot, const T *src, size_t count, const T **dst) {
+    void *p = scratch(e, slot, count * sizeof(T));
+    if (!p) return fail(e, SW_E_CUDA, "sw_verify: out of device memory for %zu bytes", count * sizeof(T));
+    if (count) {
+        CK(cudaMemcpyAsync(p, src, count * sizeof(T), cudaMemcpyHostToDevice, e->stream));
+        e->stats.h2d_bytes += count * sizeof(T);
+    }
+    *dst = reinterpret_cast<const T *>(p);
+    return 0;
+}
+
+bool offsets_ok(int n, const int64_t *off) {
+    if (off[0] < 0) return false;
+    for (int i = 0; i < n; i++) if (off[i + 1] < off[i]) return false;
+    return true;
+}
+
+// status_out[i] for the events sel[0..nsel) (every event: sel NULL, nsel = n); the others' status is 0
+int verify_impl(sw_engine *e, int n, const int32_t *sel, int nsel, const int32_t *creator, const uint8_t *sig,
+                const uint8_t *msg, const int64_t *msg_off, const uint8_t *ids, const uint8_t *wire,
+                const int64_t *wire_off, uint8_t *status_out) {
+    if (!e->keys_set) return fail(e, SW_E_ARG, "sw_verify: call sw_set_member_keys first");
+    if (!offsets_ok(n, msg_off) || !offsets_ok(n, wire_off)) return fail(e, SW_E_ARG, "sw_verify: offsets must start at >= 0 and not decrease");
+    CK(cudaSetDevice(e->device));
+    if (e->v_grid == 0) {
+        CK(cudaFuncSetAttribute(k_verify, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(swv::Precomp) * swv::COMB_ENTRIES)));
+        int per_sm = 0;
+        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_verify, SWV_THREADS, sizeof(swv::Precomp) * swv::COMB_ENTRIES));
+        e->v_grid = std::max(1, per_sm) * e->n_sm;
+    }
+    SwVerifyArgs a{};
+    a.n = nsel; a.M = e->M;
+    a.pk = e->d_vpk; a.keyok = e->d_vkeyok; a.tab = e->d_vtab;
+    if (upload(e, 0, creator, (size_t)n, &a.creator) < 0 || upload(e, 1, sig, (size_t)64 * n, &a.sig) < 0 ||
+        upload(e, 2, msg, (size_t)msg_off[n], &a.msg) < 0 || upload(e, 3, msg_off, (size_t)n + 1, &a.msg_off) < 0 ||
+        upload(e, 4, ids, (size_t)32 * n, &a.ids) < 0 || upload(e, 5, wire, (size_t)wire_off[n], &a.wire) < 0 ||
+        upload(e, 6, wire_off, (size_t)n + 1, &a.wire_off) < 0 || (sel && upload(e, 7, sel, (size_t)nsel, &a.sel) < 0))
+        return SW_E_CUDA;
+    uint8_t *d_status = reinterpret_cast<uint8_t *>(scratch(e, 8, (size_t)n));
+    if (!d_status) return fail(e, SW_E_CUDA, "sw_verify: out of device memory");
+    a.status = d_status;
+    CK(cudaMemsetAsync(d_status, 0, (size_t)n, e->stream));
+    if (nsel > 0) {
+        const int grid = std::min(e->v_grid, (nsel + SWV_THREADS - 1) / SWV_THREADS);
+        k_verify<<<grid, SWV_THREADS, sizeof(swv::Precomp) * swv::COMB_ENTRIES, e->stream>>>(a);
+        CK(cudaGetLastError());
+        e->stats.kernel_launches += 1;
+    }
+    CK(cudaMemcpyAsync(status_out, d_status, (size_t)n, cudaMemcpyDeviceToHost, e->stream));
+    CK(cudaStreamSynchronize(e->stream));
+    e->stats.d2h_bytes += n;
+    int good = 0;
+    for (int i = 0; i < n; i++) good += status_out[i] == 3;
+    return good;
+}
+}  // namespace
+
+int sw_verify(sw_engine *e, int n, const int32_t *creator, const uint8_t *sig, const uint8_t *msg, const int64_t *msg_off,
+              const uint8_t *ids, const uint8_t *wire, const int64_t *wire_off, uint8_t *status_out) {
+    if (!e || n < 0 || !msg_off || !wire_off || (n > 0 && (!creator || !sig || !ids || !status_out)) ||
+        (msg_off[n] > msg_off[0] && !msg) || (wire_off[n] > wire_off[0] && !wire))
+        return fail(e, SW_E_ARG, "bad argument");
+    return verify_impl(e, n, nullptr, n, creator, sig, msg, msg_off, ids, wire, wire_off, status_out);
+}
+
+int sw_ingest_verified(sw_engine *e, int n, const uint8_t *ids, const uint8_t *p0_ids, const uint8_t *p1_ids,
+                       const int32_t *creator, const double *t, const uint8_t *sig, const uint8_t *msg,
+                       const int64_t *msg_off, const uint8_t *wire, const int64_t *wire_off, int32_t *index_out) {
+    if (!e || n < 0 || !msg_off || !wire_off ||
+        (n > 0 && (!ids || !p0_ids || !p1_ids || !creator || !t || !sig || !index_out)) ||
+        (msg_off[n] > msg_off[0] && !msg) || (wire_off[n] > wire_off[0] && !wire))
+        return fail(e, SW_E_ARG, "bad argument");
+    if (!e->keys_set) return fail(e, SW_E_ARG, "sw_ingest_verified: call sw_set_member_keys first");
+    // only the events new to the engine are checked (ingest skips the known ones)
+    std::vector<int32_t> sel;
+    for (int i = 0; i < n; i++) {
+        Id32 k;
+        memcpy(k.data(), ids + (size_t)32 * i, 32);
+        if (e->ids.find(k) == e->ids.end()) sel.push_back(i);
+    }
+    std::vector<uint8_t> status((size_t)n, 0), rejected((size_t)n, 0);
+    if (!sel.empty()) {
+        const int rc = verify_impl(e, n, sel.data(), (int)sel.size(), creator, sig, msg, msg_off, ids, wire, wire_off, status.data());
+        if (rc < 0) return rc;
+    }
+    for (int i : sel) rejected[i] = status[i] != 3;
+    return ingest_impl(e, n, ids, p0_ids, p1_ids, creator, t, sig, rejected.data(), index_out);
 }
 
 int sw_lookup(sw_engine *e, int n, const uint8_t *ids, int32_t *index_out) {

@@ -26,6 +26,7 @@ SYMBOLS = [
     "sw_get_witness_table", "sw_get_consensus", "sw_get_transactions", "sw_get_idx", "sw_get_height",
     "sw_sync", "sw_stats", "sw_flush_l2", "sw_version", "sw_debug_counters", "sw_peer_handle", "sw_peer_connect",
     "sw_save", "sw_load", "sw_members", "sw_ingest", "sw_lookup", "sw_batch_divide_rounds",
+    "sw_set_member_keys", "sw_verify", "sw_ingest_verified",
 ]
 
 
@@ -86,6 +87,9 @@ def load_library(path: str = LIB_PATH):
     L.sw_members.argtypes = [vp]
     L.sw_ingest.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp, vp]
     L.sw_lookup.argtypes = [vp, i32, vp, vp]
+    L.sw_set_member_keys.argtypes = [vp, vp]
+    L.sw_verify.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp, vp, vp]
+    L.sw_ingest_verified.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.sw_batch_divide_rounds.argtypes = [vp, i32, vp, vp]
     L.sw_save.argtypes = [vp, C.c_char_p]
     L.sw_load.argtypes = [C.c_char_p, i32, i32, P(vp)]
@@ -95,6 +99,44 @@ def load_library(path: str = LIB_PATH):
 
 def _ptr(a: np.ndarray):
     return a.ctypes.data_as(C.c_void_p)
+
+
+def _bytes_col(buf, off, n):
+    buf = np.ascontiguousarray(np.frombuffer(buf, np.uint8) if isinstance(buf, (bytes, bytearray)) else buf, np.uint8)
+    off = np.ascontiguousarray(off, np.int64)
+    assert off.shape[0] == n + 1 and off[0] >= 0 and off[-1] <= buf.size
+    if buf.size == 0:
+        buf = np.zeros(1, np.uint8)
+    return buf, off
+
+
+def event_columns(events, member_of):
+    """The columns sw_ingest_verified / sw_verify read, from (id, Event) pairs (Event = the reference's namedtuple
+    (d, p, t, c, s)) and a public key -> member index map.  The signed bytes and the hashed bytes are serialised
+    exactly as the reference does (swirld.py:95, 99): pickle.dumps(ev[:-1]) and pickle.dumps(ev).  A creator not in
+    the map gets member -1, so its signature never verifies."""
+    import pickle
+    n = len(events)
+    zero = bytes(32)
+    ids = np.empty((n, 32), np.uint8); p0 = np.zeros((n, 32), np.uint8); p1 = np.zeros((n, 32), np.uint8)
+    creator = np.empty(n, np.int32); t = np.empty(n, np.float64); sig = np.zeros((n, 64), np.uint8)
+    msgs, wires = [], []
+    for i, (h, ev) in enumerate(events):
+        ids[i] = np.frombuffer(h, np.uint8)
+        if ev.p:
+            p0[i] = np.frombuffer(ev.p[0] or zero, np.uint8)
+            p1[i] = np.frombuffer(ev.p[1] or zero, np.uint8)
+        s = bytes(ev.s)
+        creator[i] = member_of.get(ev.c, -1) if len(s) == 64 else -1     # (a signature of another length never verifies)
+        t[i] = ev.t
+        sig[i, :min(64, len(s))] = np.frombuffer(s[:64], np.uint8)
+        msgs.append(pickle.dumps(ev[:-1]))
+        wires.append(pickle.dumps(ev))
+    msg_off = np.zeros(n + 1, np.int64); msg_off[1:] = np.cumsum([len(m) for m in msgs])
+    wire_off = np.zeros(n + 1, np.int64); wire_off[1:] = np.cumsum([len(w) for w in wires])
+    return {"ids": ids, "p0_ids": p0, "p1_ids": p1, "creator": creator, "t": t, "sig": sig,
+            "msg": np.frombuffer(b"".join(msgs), np.uint8), "msg_off": msg_off,
+            "wire": np.frombuffer(b"".join(wires), np.uint8), "wire_off": wire_off}
 
 
 class Engine:
@@ -186,6 +228,43 @@ class Engine:
         sig = np.ascontiguousarray(sig, np.uint8).reshape(n, 64)
         out = np.empty(n, np.int32)
         m = self._chk(self._lib.sw_ingest(self._h, n, _ptr(ids), _ptr(p0_ids), _ptr(p1_ids), _ptr(creator), _ptr(t), _ptr(sig), _ptr(out)))
+        return out, m
+
+    # -- is_valid_event's crypto checks on the GPU (Ed25519 signature, BLAKE2b id)
+    def set_member_keys(self, pks) -> int:
+        """The members' 32-byte public keys in member order; returns how many of them libsodium would reject."""
+        pk = np.ascontiguousarray(np.frombuffer(b"".join(bytes(k) for k in pks), np.uint8)
+                                  if not isinstance(pks, np.ndarray) else pks, np.uint8).reshape(-1, 32)
+        assert pk.shape[0] == self.M
+        return self._chk(self._lib.sw_set_member_keys(self._h, _ptr(pk)))
+
+    def verify(self, creator, sig, msg, msg_off, ids, wire, wire_off):
+        """sw_verify: per event, bit 0 = the signature verifies, bit 1 = the id is BLAKE2b-256 of the wire bytes."""
+        creator = np.ascontiguousarray(creator, np.int32)
+        n = creator.shape[0]
+        sig = np.ascontiguousarray(sig, np.uint8).reshape(n, 64)
+        ids = np.ascontiguousarray(ids, np.uint8).reshape(n, 32)
+        msg, msg_off = _bytes_col(msg, msg_off, n)
+        wire, wire_off = _bytes_col(wire, wire_off, n)
+        out = np.zeros(n, np.uint8)
+        self._chk(self._lib.sw_verify(self._h, n, _ptr(creator), _ptr(sig), _ptr(msg), _ptr(msg_off), _ptr(ids),
+                                      _ptr(wire), _ptr(wire_off), _ptr(out)))
+        return out
+
+    def ingest_verified(self, ids, p0_ids, p1_ids, creator, t, sig, msg, msg_off, wire, wire_off):
+        """sw_ingest_verified: ingest() that first checks the new events' signatures and ids; returns (index, appended)."""
+        ids = np.ascontiguousarray(ids, np.uint8).reshape(-1, 32)
+        n = ids.shape[0]
+        p0_ids = np.ascontiguousarray(p0_ids, np.uint8).reshape(n, 32)
+        p1_ids = np.ascontiguousarray(p1_ids, np.uint8).reshape(n, 32)
+        creator = np.ascontiguousarray(creator, np.int32); t = np.ascontiguousarray(t, np.float64)
+        sig = np.ascontiguousarray(sig, np.uint8).reshape(n, 64)
+        msg, msg_off = _bytes_col(msg, msg_off, n)
+        wire, wire_off = _bytes_col(wire, wire_off, n)
+        out = np.empty(n, np.int32)
+        m = self._chk(self._lib.sw_ingest_verified(self._h, n, _ptr(ids), _ptr(p0_ids), _ptr(p1_ids), _ptr(creator),
+                                                   _ptr(t), _ptr(sig), _ptr(msg), _ptr(msg_off), _ptr(wire),
+                                                   _ptr(wire_off), _ptr(out)))
         return out, m
 
     def lookup(self, ids):
